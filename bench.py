@@ -1,6 +1,6 @@
 """bench.py — denoised latent frames/sec of the SVI clip-denoising hot path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg2|cfg3|cfg4|cfg5|cfg1|tiny]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg2|cfg3|cfg4|cfg5|cfg1|tiny] [--dump-outputs DIR]
 
 Default workload cfg2 = BASELINE.json configs[1] (the configuration the metric is quoted on): a "step" is ONE
 flow-matching denoise step of the clip — two Wan-DiT forwards (classifier-free guidance) + the fused CFG/Euler update —
@@ -265,7 +265,14 @@ def main():
     ap.add_argument("--no-vae", action="store_true", help="skip the clip-boundary VAE leg (decode 21->81 frames, encode 81 frames)")
     ap.add_argument("--no-sp-parity", action="store_true", help="N>1: skip the plan-vs-single-rank check before the timed run")
     ap.add_argument("--clips", type=int, default=10, help="cfg4: clips in the chain")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float32): "
+                    "the updated latents and, on one GPU, the conditional / unconditional velocity fields; inputs are seeded, "
+                    "so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.workload not in WORKLOADS):
+        ap.error("--dump-outputs applies to the native DiT workloads (" + ", ".join(WORKLOADS) + ")")
     if args.workload == "cfg4":
         from tools import clip_loop_bench
         return clip_loop_bench.main_from_bench(args)
@@ -380,6 +387,18 @@ def main():
     e1.record()
     sync()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # taken before anything else runs a step: the steps below reuse lat, v_c and v_u.  The latents are replicated on every
+        # rank; v_c / v_u hold the full velocity fields only on one GPU.  Largest workload (cfg3): 3 x 19.4 MB.
+        outs = {"latents": lat}
+        if world == 1:
+            outs.update(velocity_cond=v_c, velocity_uncond=v_u)
+        if rank == 0:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, t in outs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), t.float().cpu().numpy())
+        sync()
     ms = e0.elapsed_time(e1)
     launches = eng.k.launches - launches0
     attn_ms = [a.elapsed_time(b) for a, b in eng.attn_events]

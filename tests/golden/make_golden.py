@@ -183,8 +183,15 @@ def golden_talk(dit_mod):
         tokens = model.audio_proj(first, latter)
         out = model(inp["x"], ts, inp["context"], clip_feature=inp["clip_feature"], y=inp["y"], audio_embed_tuple=(first, latter))
         base = model(inp["x"], ts, inp["context"], clip_feature=inp["clip_feature"], y=inp["y"])
+    # the first frame's windows are a gather of the seeded audio features: stored as the (video frame, window) each
+    # [12, 768] row comes from, plus a checksum of the features, which keeps the fixture under 1 MB
+    feats = audio[0].flatten(2)                 # [video frames, windows, 12 * 768]
+    idx = [(feats == r).all(-1).nonzero() for r in first.reshape(-1, feats.shape[-1])]
+    assert all(len(i) == 1 for i in idx)
+    first_src = torch.cat(idx).reshape(first.shape[1:-2] + (2,)).numpy()
     np.savez_compressed(os.path.join(HERE, "dit_tiny_talk.npz"), out=out.numpy(), out_no_audio=base.numpy(),
-                        audio_tokens=tokens.numpy(), first=first.numpy(), latter=latter.numpy(), fhw=np.array([f, h, w]),
+                        audio_tokens=tokens.numpy(), first_src=first_src, latter=latter.numpy(),
+                        audio_checksum=np.float64(audio.double().sum().item()), fhw=np.array([f, h, w]),
                         seed=np.array(5), ctx_len=np.array(24), timestep=ts.numpy())
     print("talk: out", tuple(out.shape), "audio tokens", tuple(tokens.shape), "max|out - no_audio|", float((out - base).abs().max()))
 

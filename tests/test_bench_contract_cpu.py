@@ -25,6 +25,15 @@ def test_reference_arm_prints_the_contract_line():
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
 
 
+def test_bench_rejects_arguments_it_cannot_honour(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)],
+                  ["--workload", "cfg5", "--dump-outputs", str(tmp_path)]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tiny"] + extra,
+                           capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 2 and "error:" in r.stderr, extra
+    assert not os.listdir(tmp_path)
+
+
 def test_native_arm_refuses_to_run_without_a_gpu():
     import torch
     if torch.cuda.is_available():
