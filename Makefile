@@ -4,7 +4,7 @@ PKG := stable-video-infinity_b200
 CSRC := $(PKG)/csrc
 LIB := $(PKG)/lib/libsvi_b200.so
 NVFLAGS := -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC
-SRCS := $(CSRC)/runtime.cu $(CSRC)/gemm_tcgen05.cu $(CSRC)/gemm2_tcgen05.cu $(CSRC)/attn_tcgen05.cu $(CSRC)/sp_exchange.cu $(CSRC)/elementwise.cu $(CSRC)/conv3d_tcgen05.cu $(CSRC)/conv3d2_tcgen05.cu $(CSRC)/vae_elementwise.cu $(CSRC)/encoder_kernels.cu
+SRCS := $(CSRC)/runtime.cu $(CSRC)/gemm_tcgen05.cu $(CSRC)/gemm2_tcgen05.cu $(CSRC)/attn_tcgen05.cu $(CSRC)/sp_exchange.cu $(CSRC)/elementwise.cu $(CSRC)/conv3d_tcgen05.cu $(CSRC)/conv3d2_tcgen05.cu $(CSRC)/vae_elementwise.cu $(CSRC)/encoder_kernels.cu $(CSRC)/audio_kernels.cu
 OBJS := $(patsubst $(CSRC)/%.cu,build/%.o,$(SRCS))
 
 all: $(LIB)

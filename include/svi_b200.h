@@ -350,6 +350,43 @@ int svi_attn_small(const void* Q, int64_t ldq, const void* K, int64_t ldk, const
                    int64_t ldo, int32_t Lq, int32_t Lk, int32_t num_heads, int32_t head_dim, float scale,
                    const float* bias_table, const int32_t* bucket, const int32_t* key_mask, void* stream);
 
+/*
+ * ---- wav2vec2 audio encoder of SVI-Talk (group-norm / post-LN variant, chinese-wav2vec2-base) ------------------------
+ * Reference: utils/audio_process.py:18-41 (get_embedding) running utils/src/audio_analysis/wav2vec2.py:13-64 on
+ * transformers' modeling_wav2vec2.  Activations are channels-last.  Convolutions 2-7 are svi_gemm_bf16 calls on strided
+ * views of the previous activation (K = k*C, lda = s*C; for k = 3 a two-pass split, see DESIGN.md §4); the feature
+ * projection, q|k|v, out-projection and feed-forward layers are svi_gemm_bf16, the attention svi_attn_small (head_dim 64).
+ *
+ * svi_audio_conv0_gn_gelu   out bf16 [T0, C] = GELU_erf(GroupNorm_C(conv1d(wav, w[C, k], stride))), T0 = (n - k)/stride + 1,
+ *                           per-channel statistics over the whole time axis (Wav2Vec2GroupNormConvLayer: conv 1->512, k 10,
+ *                           s 5, no bias; nn.GroupNorm(512, 512, eps, affine)).  Two passes over the waveform: per-block fp64
+ *                           partial sums, merged in block order, then the conv is recomputed and normalised; the fp32 conv
+ *                           output is never stored and nothing is accumulated with atomics.  workspace: 16-byte aligned,
+ *                           svi_audio_conv0_workspace_bytes(n, C, k, stride) bytes; on completion its first 2*C floats
+ *                           hold the channel means and 1/sqrt(var + eps).  C % 32 == 0, C <= 1024, k <= 16.
+ * svi_audio_interp_layernorm  y bf16 [S, C] = LayerNorm(F.interpolate(x^T, S, mode='linear', align_corners=True)^T)
+ *                           * gamma + beta, x f32 [T_in, C] (torch_utils.py:16-19 + Wav2Vec2FeatureProjection.layer_norm).
+ * svi_audio_pos_conv        out f32 [S, D] = x + GELU_erf(conv1d(x, groups, k, padding k/2)[:S] + bias)
+ *                           (Wav2Vec2PositionalConvEmbedding incl. Wav2Vec2SamePadLayer, plus the residual add of
+ *                           Wav2Vec2Encoder.forward); w_packed f32 [groups][k][cg][cg] with [g][j][c][o] = w[g*cg + o, c, j]
+ *                           (weight norm folded on the host), cg = D / groups a multiple of 8 and <= 64, k even.
+ *                           out must not alias x.
+ * svi_layernorm_f32x2       y f32 [M, ldy] and y_bf16 bf16 [M, D] (contiguous) = LayerNorm(x [M, ldx]) * gamma + beta:
+ *                           the post-LN LayerNorms of Wav2Vec2EncoderLayer, whose output is both the next residual (fp32,
+ *                           or a slot of the stacked [S, layers, D] result when ldy = layers*D) and the next GEMM's A.
+ *                           y may alias x.
+ */
+size_t svi_audio_conv0_workspace_bytes(int64_t n_samples, int32_t C, int32_t k, int32_t stride);
+int svi_audio_conv0_gn_gelu(const float* wav, int64_t n_samples, const float* w, int32_t C, int32_t k, int32_t stride,
+                            const float* gamma, const float* beta, float eps, void* out_bf16, void* workspace,
+                            size_t workspace_bytes, void* stream);
+int svi_audio_interp_layernorm(const float* x, int32_t T_in, int32_t C, int32_t S, const float* gamma, const float* beta,
+                               float eps, void* y_bf16, void* stream);
+int svi_audio_pos_conv(const float* x, int32_t S, int32_t D, int32_t groups, int32_t k, const float* w_packed,
+                       const float* bias, float* out, void* stream);
+int svi_layernorm_f32x2(const float* x, int64_t ldx, int32_t M, int32_t D, float eps, const float* gamma,
+                        const float* beta, float* y, int64_t ldy, void* y_bf16, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -97,6 +97,11 @@ SIGNATURES = {
     "svi_vae_to_planar": (_i32, [_vp, _i64, _i32, _i64, _vp, _vp, _i32, _vp, _i64, _vp]),
     "svi_softmax_rows": (_i32, [_vp, _i32, _i32, _i64, _f32, _vp, _i64, _vp]),
     "svi_frames_to_uint8": (_i32, [_vp, _i64, _i64, _vp, _vp]),
+    "svi_audio_conv0_workspace_bytes": (_c.c_size_t, [_i64, _i32, _i32, _i32]),
+    "svi_audio_conv0_gn_gelu": (_i32, [_vp, _i64, _vp, _i32, _i32, _i32, _vp, _vp, _f32, _vp, _vp, _c.c_size_t, _vp]),
+    "svi_audio_interp_layernorm": (_i32, [_vp, _i32, _i32, _i32, _vp, _vp, _f32, _vp, _vp]),
+    "svi_audio_pos_conv": (_i32, [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),
+    "svi_layernorm_f32x2": (_i32, [_vp, _i64, _i32, _i32, _f32, _vp, _vp, _vp, _i64, _vp, _vp]),
 }
 
 _lib = None
@@ -606,3 +611,60 @@ def softmax_rows(s, N, scale, p):
                                  _ptr(p, torch.bfloat16, "p"), _rowmajor(p, "p"), _stream())
     _check(rc, "svi_softmax_rows")
     return p
+
+
+# --------------------------------------------------------------------------------------------- wav2vec2 audio encoder
+def audio_conv0_gn_gelu(wav, w, gamma, beta, eps, stride, out, workspace=None):
+    """out bf16 [T0, C] = GELU(GroupNorm_C(conv1d(wav f32 [n], w f32 [C, k], stride))) (svi_audio_conv0_gn_gelu).
+    Returns the workspace (uint8, CUDA); its first 2*C floats hold the channel means and 1/sqrt(var + eps)."""
+    C, k = w.shape
+    n = wav.numel()
+    T0 = (n - k) // stride + 1
+    if not (wav.is_contiguous() and w.is_contiguous() and out.is_contiguous()) or tuple(out.shape) != (T0, C):
+        raise RuntimeError(f"svi_b200.audio_conv0_gn_gelu: contiguous wav [n], w [C,k] and out [{T0},{C}] required")
+    nbytes = int(load().svi_audio_conv0_workspace_bytes(n, C, k, stride))
+    if workspace is None or workspace.numel() < nbytes:
+        workspace = torch.empty(nbytes, dtype=torch.uint8, device=wav.device)
+    rc = load().svi_audio_conv0_gn_gelu(_ptr(wav, torch.float32, "wav"), n, _ptr(w, torch.float32, "w"), C, k, stride,
+                                        _ptr(gamma, torch.float32, "gamma"), _ptr(beta, torch.float32, "beta"), float(eps),
+                                        _ptr(out, torch.bfloat16, "out"), _ptr(workspace, name="workspace"), workspace.numel(),
+                                        _stream())
+    _check(rc, "svi_audio_conv0_gn_gelu")
+    return workspace
+
+
+def audio_interp_layernorm(x, gamma, beta, eps, out):
+    """out bf16 [S, C] = LayerNorm(linear interpolation (align_corners) of x f32 [T_in, C] to S rows) * gamma + beta."""
+    T_in, C = x.shape
+    if not x.is_contiguous() or not out.is_contiguous() or out.shape[1] != C:
+        raise RuntimeError("svi_b200.audio_interp_layernorm: contiguous x [T_in, C] and out [S, C] required")
+    rc = load().svi_audio_interp_layernorm(_ptr(x, torch.float32, "x"), T_in, C, out.shape[0], _ptr(gamma, torch.float32, "gamma"),
+                                           _ptr(beta, torch.float32, "beta"), float(eps), _ptr(out, torch.bfloat16, "out"), _stream())
+    _check(rc, "svi_audio_interp_layernorm")
+    return out
+
+
+def audio_pos_conv(x, w_packed, bias, groups, out):
+    """out f32 [S, D] = x + GELU(grouped conv1d(x, k, padding k/2)[:S] + bias); w_packed f32 [groups, k, cg, cg]."""
+    S, D = x.shape
+    g, k, cg, cg2 = w_packed.shape
+    if g != groups or cg != cg2 or g * cg != D or not (x.is_contiguous() and out.is_contiguous() and w_packed.is_contiguous()) \
+            or out.shape != x.shape:
+        raise RuntimeError("svi_b200.audio_pos_conv: contiguous x / out [S, D] and w_packed [groups, k, D/groups, D/groups] required")
+    rc = load().svi_audio_pos_conv(_ptr(x, torch.float32, "x"), S, D, groups, k, _ptr(w_packed, torch.float32, "w_packed"),
+                                   _ptr(bias, torch.float32, "bias"), _ptr(out, torch.float32, "out"), _stream())
+    _check(rc, "svi_audio_pos_conv")
+    return out
+
+
+def layernorm_f32x2(x, gamma, beta, eps, out, out_bf16):
+    """out f32 [M, D] (row-strided view allowed) and out_bf16 contiguous bf16 [M, D] = LayerNorm(x) * gamma + beta."""
+    M, D = x.shape
+    if tuple(out.shape) != (M, D) or tuple(out_bf16.shape) != (M, D) or not out_bf16.is_contiguous():
+        raise RuntimeError("svi_b200.layernorm_f32x2: out [M, D] and contiguous out_bf16 [M, D] required")
+    rc = load().svi_layernorm_f32x2(_ptr(x, torch.float32, "x"), _rowmajor(x, "x"), M, D, float(eps),
+                                    _ptr(gamma, torch.float32, "gamma"), _ptr(beta, torch.float32, "beta"),
+                                    _ptr(out, torch.float32, "out"), _rowmajor(out, "out"), _ptr(out_bf16, torch.bfloat16, "out_bf16"),
+                                    _stream())
+    _check(rc, "svi_layernorm_f32x2")
+    return out

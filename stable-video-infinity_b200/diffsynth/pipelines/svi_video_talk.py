@@ -8,9 +8,13 @@ into a first-frame window and per-latent-frame windows (`preprocess_audio`, :432
     v = v_uncond + s_text * (v_cond - v_drop_text) + s_audio * (v_drop_text - v_uncond)
 
 with v_cond (prompt, audio), v_drop_text (negative prompt, audio), v_uncond (negative prompt, silent audio).
-The wav2vec2 feature extractor is an external model (`utils/src/audio_analysis` in the reference, not part of diffsynth):
-pass its output as `audio_embed`; `audio_path` alone raises.
+The window features come from `audio_path` (a WAV file) through the native wav2vec2 encoder
+(utils/src/audio_analysis/wav2vec2.py, loaded lazily from `wav2vec_path`, default ./weights/chinese-wav2vec2-base/ as in the
+reference), or are passed in directly as `audio_embed`.  The embedding of the whole file is kept on the device for the
+next call with the same file (keyed by real path, size and mtime), so chained clips encode their audio once.
 """
+import os
+
 import torch
 from PIL import Image
 from tqdm import tqdm
@@ -53,6 +57,8 @@ class SVITalkVideoPipeline(SVIVideoPipeline):
     def __init__(self, device="cuda", torch_dtype=torch.float16, tokenizer_path=None, wav2vec_path=None, is_test=False):
         super().__init__(device=device, torch_dtype=torch_dtype, tokenizer_path=tokenizer_path, is_test=is_test)
         self.wav2vec_path = wav2vec_path
+        self.wav2vec_feature_extractor, self.audio_encoder = None, None
+        self._audio_cache = None          # ((realpath, size, mtime_ns), [S, layers, 768] f32 on the device)
 
     @staticmethod
     def from_model_manager(model_manager, torch_dtype=None, device=None, use_usp=False, is_test=False, wav2vec_path=None):
@@ -64,10 +70,35 @@ class SVITalkVideoPipeline(SVIVideoPipeline):
             pipe.enable_usp()
         return pipe
 
+    def load_audio_encoder(self):
+        """custom_init (reference :26-30): feature extractor + encoder from `wav2vec_path`, on first use."""
+        if self.audio_encoder is None:
+            from utils.src.audio_analysis.wav2vec2 import Wav2Vec2FeatureExtractor, Wav2Vec2Model
+            path = self.wav2vec_path if self.wav2vec_path is not None else "./weights/chinese-wav2vec2-base/"
+            if not os.path.isdir(path):
+                raise FileNotFoundError(f"wav2vec2 checkpoint directory not found: {os.path.abspath(path)} "
+                                        f"(pass wav2vec_path=, or audio_embed= with precomputed window features)")
+            self.wav2vec_feature_extractor = Wav2Vec2FeatureExtractor.from_pretrained(path, local_files_only=True)
+            self.audio_encoder = Wav2Vec2Model.from_pretrained(path, local_files_only=True)
+        return self.wav2vec_feature_extractor, self.audio_encoder
+
+    def audio_embedding(self, audio_path):
+        """[S, layers, 768] f32 on the device for the whole file; recomputed only when the file changes."""
+        from utils.audio_process import audio_prepare_single, embedding_device
+        st = os.stat(audio_path)
+        key = (os.path.realpath(audio_path), st.st_size, st.st_mtime_ns)
+        if self._audio_cache is None or self._audio_cache[0] != key:
+            fe, enc = self.load_audio_encoder()
+            self._audio_cache = None
+            emb = embedding_device(audio_prepare_single(audio_path), fe, enc, device=self.device)
+            self._audio_cache = (key, emb)
+        return self._audio_cache[1]
+
     def get_audio_embedding(self, audio_path, num_frames, audio_start_idx=0):
-        raise NotImplementedError(
-            "svi_b200: wav2vec2 feature extraction is not part of this package (the reference uses its own "
-            "utils/src/audio_analysis model); pass the [1, num_frames, 5, 12, 768] window features as audio_embed=")
+        """reference :412-430: [1, num_frames, 5, layers, 768] window features of frames audio_start_idx .. + num_frames,
+        window rows clamped to the audio; every rank of a use_usp group computes the same bits (no atomics on the path)."""
+        from utils.audio_process import cut_windows
+        return cut_windows(self.audio_embedding(audio_path), num_frames, audio_start_idx)
 
     def preprocess_audio(self, audio_embed, audio_window=5, vae_scale=4):
         first, latter = preprocess_audio(audio_embed, audio_window, vae_scale)

@@ -33,3 +33,19 @@ def vae_encode_flops(t_lat, H, W):
 def vae_min_bytes(t_lat, h, w):
     """Minimal conv in+out traffic (bf16) of the VAE decoder per clip: 8.5 GB per latent frame at 480p (60x104), SURVEY §8d."""
     return 8.5e9 * t_lat * (h * w) / 6240.0
+
+
+def wav2vec_flops(n_samples, cfg, sr=16000):
+    """FLOPs of one wav2vec2 embedding of n_samples (multiply-add = 2), by stage: conv stack, positional conv, GEMMs
+    (feature projection + per layer q|k|v, out-projection, feed-forward) and attention (QK^T and PV)."""
+    T, cin, conv = n_samples, 1, 0
+    for c, k, s in zip(cfg["conv_dim"], cfg["conv_kernel"], cfg["conv_stride"]):
+        T = (T - k) // s + 1
+        conv += 2 * T * c * cin * k
+        cin = c
+    S = int(n_samples / sr * 25)
+    D, I, L = cfg["hidden_size"], cfg["intermediate_size"], cfg["num_hidden_layers"]
+    gemm = 2 * S * cin * D + L * 2 * S * (4 * D * D + 2 * D * I)
+    pos = 2 * S * D * (D // cfg["num_conv_pos_embedding_groups"]) * cfg["num_conv_pos_embeddings"]
+    attn = L * 4 * S * S * D
+    return dict(conv=conv, pos_conv=pos, gemm=gemm, attention=attn)
